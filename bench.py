@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 5 --warmup 3
     python bench.py --impl reference --steps 3 --warmup 1      # the CPU arm (reference modules / oracle port)
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs /tmp/out   # + the last timed step's loss and gradients
 
 One "step" = x -> ViTEncoder -> pre_quant -> VectorQuantizer -> post_quant -> ViTDecoder ->
 loss = mean((rec-x)^2) + qloss -> backward, fp32 parameters, no optimizer step (SURVEY.md
@@ -23,6 +24,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
+
+DUMP_BUDGET_BYTES = 64 * 2 ** 20
+DUMP_SAMPLE = 32768                     # elements kept of a larger gradient
 
 METRIC = "images/sec (256x256) ViT-VQGAN fwd+bwd"
 UNIT = "images/s"
@@ -273,6 +278,32 @@ def vq_block(dev, peaks):
     return res
 
 
+def dump_outputs(out_dir, loss, named_params):
+    """what the caller of one timed step receives -- the loss and every parameter's gradient -- as float32 .npy files:
+    loss.npy and grad.<parameter name>.npy.  A gradient of more than DUMP_SAMPLE elements is stored as the elements at
+    DUMP_SAMPLE fixed positions (a permutation seeded by the parameter name, sorted), so that two builds of the project can
+    be compared output for output."""
+    import zlib
+
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().cpu().numpy()}
+    for name, p in named_params:
+        if p.grad is None:
+            continue
+        flat = p.grad.detach().float().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randperm(flat.numel(), generator=g)[:DUMP_SAMPLE].sort().values
+            flat = flat[idx.to(flat.device)]
+        arrays["grad." + name] = flat.cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BUDGET_BYTES, f"--dump-outputs: {total} bytes exceed the {DUMP_BUDGET_BYTES}-byte budget"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -288,7 +319,11 @@ def main():
     ap.add_argument("--no-fuse-pos", action="store_true", help="keep post_quant and the decoder's positional add separate")
     ap.add_argument("--extras", default="vq,secondary,eager,cpu",
                     help="comma list of the 1-GPU extra blocks to measure after the timed regions: vq, secondary, eager, cpu ('' = none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's loss and parameter gradients (sampled, float32) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -432,11 +467,14 @@ def main():
         if i + 1 < args.steps:
             with torch.cuda.stream(copy_stream):       # step i+1's images travel while step i computes
                 nxt = host_imgs[(i + 1) % 2].to(dev, non_blocking=True)
-        last = float(step(x).item())                   # device -> host read of the step's result
+        loss = step(x)
+        last = float(loss.item())                      # device -> host read of the step's result
     ev3.record()
     barrier()
     ms_e2e = ev2.elapsed_time(ev3)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, sorted(model.named_parameters()))
 
     t = torch.tensor([ms_total, ms_e2e, comm_ms], device=dev, dtype=torch.float64)
     per_rank = comm_rank = None

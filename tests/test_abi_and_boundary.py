@@ -126,63 +126,88 @@ def test_init_distributions_follow_reference():
     assert abs(vq.embedding.weight.std().item() - 1.0) < 0.05
 
 
-REF = "/root/reference"
+def _vitvqgan_stand_in():
+    """a module laid out like the reference's stage1/vitvqgan.py as far as this package touches it: module-level names
+    Encoder / Decoder / VectorQuantizer that ViTVQ.__init__ looks up when it runs, plain nn.Linear pre/post_quant, and a
+    training_step that runs the whole autoencoder and hands the reconstruction to the loss with the optimizer index"""
+    import types
+
+    mod = types.ModuleType("vitvqgan_stand_in")
+
+    class ViTVQ(torch.nn.Module):
+        def __init__(self, image_size, patch_size, encoder, decoder, quantizer, loss):
+            super().__init__()
+            self.image_key, self.loss, self.global_step = "image", loss, 0
+            self.encoder = mod.Encoder(image_size=image_size, patch_size=patch_size, **encoder)
+            self.decoder = mod.Decoder(image_size=image_size, patch_size=patch_size, **decoder)
+            self.quantizer = mod.VectorQuantizer(**quantizer)
+            self.pre_quant = torch.nn.Linear(encoder["dim"], quantizer["embed_dim"])
+            self.post_quant = torch.nn.Linear(quantizer["embed_dim"], decoder["dim"])
+
+        def encode(self, x):
+            quant, qloss, _ = self.quantizer(self.pre_quant(self.encoder(x)))
+            return quant, qloss
+
+        def decode(self, quant):
+            return self.decoder(self.post_quant(quant))
+
+        def forward(self, x):
+            quant, qloss = self.encode(x)
+            return self.decode(quant), qloss
+
+        def training_step(self, batch, batch_idx, optimizer_idx=0):
+            x = batch[self.image_key]
+            xrec, qloss = self(x)
+            loss, _ = self.loss(qloss, x, xrec, optimizer_idx, self.global_step, batch_idx,
+                                last_layer=self.decoder.get_last_layer(), split="train")
+            return loss
+
+    mod.ViTVQ = ViTVQ
+    return mod
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
-def test_unchanged_lightning_module_constructs_with_patched_classes(monkeypatch):
-    """ViTVQ from the reference's vitvqgan.py, unedited, built on top of the replacement classes
-    (stub pytorch_lightning / omegaconf, which are not installed here; SURVEY.md section 8c)."""
-    import importlib.util
+def test_unchanged_lightning_module_constructs_with_patched_classes(golden_dir, monkeypatch):
+    """a ViTVQ built on the replacement classes has the state-dict keys and shapes of the reference's own ViTVQ
+    (stage1/vitvqgan.py built from its own classes: tests/golden/ref_modules.npz, oracle/gen_golden_live.py), whether the
+    names resolve through install_as_reference_modules() or are rebound by patch(); SURVEY.md section 8c"""
     import sys
     import types
 
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        monkeypatch.setitem(sys.modules, name, m)
-        return m
-
-    class AttrDict(dict):
-        __getattr__ = dict.__getitem__
-
-    stub("omegaconf", OmegaConf=AttrDict)
-    pl = stub("pytorch_lightning", LightningModule=torch.nn.Module)
-    for pkg in ("enhancing", "enhancing.modules", "enhancing.modules.stage1", "enhancing.utils"):
-        stub(pkg).__path__ = []
-    stub("enhancing.utils.general", initialize_from_config=lambda cfg: torch.nn.Identity())
-    etb.install_as_reference_modules()
+    from oracle.gen_golden_live import VITVQ_KW as kw
+    from oracle.seeded import parse_shapes
+    want = parse_shapes(np.load(os.path.join(golden_dir, "ref_modules.npz"))["vitvq.shapes"])
     for n in ("enhancing.modules.stage1.layers", "enhancing.modules.stage1.quantizers"):
-        monkeypatch.setitem(sys.modules, n, sys.modules[n])
-    spec = importlib.util.spec_from_file_location("enhancing.modules.stage1.vitvqgan",
-                                                  os.path.join(REF, "enhancing", "modules", "stage1", "vitvqgan.py"))
-    mod = importlib.util.module_from_spec(spec)
-    monkeypatch.setitem(sys.modules, spec.name, mod)
-    spec.loader.exec_module(mod)
+        monkeypatch.delitem(sys.modules, n, raising=False)
+    etb.install_as_reference_modules()
+    mod = _vitvqgan_stand_in()
+    # what the reference's `from .layers import ViTEncoder as Encoder, ...` binds once the package's classes are installed
+    mod.Encoder = sys.modules["enhancing.modules.stage1.layers"].ViTEncoder
+    mod.Decoder = sys.modules["enhancing.modules.stage1.layers"].ViTDecoder
+    mod.VectorQuantizer = sys.modules["enhancing.modules.stage1.quantizers"].VectorQuantizer
     assert mod.Encoder is etb.ViTEncoder and mod.Decoder is etb.ViTDecoder and mod.VectorQuantizer is etb.VectorQuantizer
-    enc = AttrDict(dim=64, depth=1, heads=2, mlp_dim=64)
-    model = mod.ViTVQ(image_key="image", image_size=32, patch_size=8, encoder=enc, decoder=enc,
-                      quantizer=AttrDict(embed_dim=32, n_embed=128), loss=AttrDict())
+
+    def build():
+        return mod.ViTVQ(kw["image_size"], kw["patch_size"], kw["encoder"], kw["encoder"], kw["quantizer"], loss=torch.nn.Identity())
+    model = build()
     assert isinstance(model.encoder, etb.ViTEncoder) and isinstance(model.quantizer, etb.VectorQuantizer)
+    assert {k: tuple(v.shape) for k, v in model.state_dict().items()} == want
     keys = set(model.state_dict())
-    assert {"encoder.en_pos_embedding", "decoder.to_pixel.1.weight", "quantizer.embedding.weight", "pre_quant.weight"} <= keys
     # patch() on an already-imported module rebinds the same three names
     mod.Encoder = None
     etb.patch(mod)
     assert mod.Encoder is etb.ViTEncoder
     # ... and makes every ViTVQ built afterwards carry QuantLinear pre/post_quant that share the nn.Linear parameters
-    # and state-dict keys (vitvqgan.py:38-39); patching twice does not wrap twice
+    # and state-dict keys; patching twice does not wrap twice
     etb.patch(mod)
     assert mod.ViTVQ.__init__.__wrapped__.__name__ == "__init__" and not hasattr(mod.ViTVQ.__init__.__wrapped__, "__wrapped__")
-    model2 = mod.ViTVQ(image_key="image", image_size=32, patch_size=8, encoder=enc, decoder=enc,
-                       quantizer=AttrDict(embed_dim=32, n_embed=128), loss=AttrDict())
+    model2 = build()
     assert isinstance(model2.pre_quant, etb.QuantLinear) and isinstance(model2.post_quant, etb.QuantLinear)
     assert set(model2.state_dict()) == keys
     model2.load_state_dict(model.state_dict(), strict=True)
     plain = torch.nn.Linear(64, 32)
     fused = etb.QuantLinear.from_linear(plain)
     assert fused.weight is plain.weight and fused.bias is plain.bias and isinstance(fused, torch.nn.Linear)
-    # opt-in: the discriminator step's forward (optimizer_idx == 1, vitvqgan.py:116-127) runs without an autograd graph
+    # opt-in: the discriminator step's forward (optimizer_idx == 1) runs without an autograd graph
     seen = []
 
     class Probe(torch.nn.Module):                                # stands in for VQLPIPSWithDiscriminator
@@ -190,7 +215,6 @@ def test_unchanged_lightning_module_constructs_with_patched_classes(monkeypatch)
             seen.append((optimizer_idx, xrec.requires_grad, torch.is_grad_enabled()))
             key = "train/total_loss" if optimizer_idx == 0 else "train/disc_loss"
             return xrec.sum() * 0 + 1.0, {key: torch.tensor(1.0)}
-
 
     class Tiny(mod.ViTVQ):                                       # no GPU here: swap the heavy parts for CPU stand-ins
         def __init__(self):
@@ -201,7 +225,6 @@ def test_unchanged_lightning_module_constructs_with_patched_classes(monkeypatch)
             self.global_step = 0
         encode = lambda self, x: (self.lin(x), x.sum() * 0)
         decode = lambda self, q: q
-        log = log_dict = lambda self, *a, **k: None
 
     etb.detach_discriminator_forward(Tiny)
     etb.detach_discriminator_forward(Tiny)                       # idempotent
@@ -238,58 +261,29 @@ def test_fuse_post_quant_pos_keeps_the_checkpoint_abi():
         etb.fuse_post_quant_pos(torch.nn.Linear(2, 2))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
-def test_unchanged_cond_transformer_constructs_with_patch_stage2(monkeypatch):
-    """CondTransformer from the reference's stage2/transformer.py, unedited: after `etb.patch_stage2` its YAML-style
-    `transformer.target: enhancing.modules.stage2.layers.GPT` resolves (by the reference's own get_obj_from_str logic,
-    utils/general.py:29-41) to this package's GPT; `configure_optimizers` (transformer.py:131-166) sorts its parameters
-    into decay / no-decay sets without leftovers."""
-    import importlib
-    import importlib.util
-    import sys
+def test_unchanged_cond_transformer_constructs_with_patch_stage2(golden_dir):
+    """after `etb.patch_stage2` a YAML-style `transformer.target: enhancing.modules.stage2.layers.GPT` resolves by attribute
+    lookup (the reference's get_obj_from_str, utils/general.py:29-41) to this package's GPT, whose parameters carry the
+    names and owning module kinds (Linear / LayerNorm / Embedding / other) of the reference's own GPT
+    (tests/golden/ref_modules.npz, oracle/gen_golden_live.py): what the reference's CondTransformer.configure_optimizers
+    (stage2/transformer.py:131-166) sorts into decay / no-decay sets"""
     import types
 
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        monkeypatch.setitem(sys.modules, name, m)
-        return m
-
-    class AttrDict(dict):
-        __getattr__ = dict.__getitem__
-
-    def initialize_from_config(config):                      # utils/general.py:29-41, verbatim semantics
-        module, cls = config["target"].rsplit(".", 1)
-        return getattr(importlib.import_module(module), cls)(**config.get("params", dict()))
-
-    stub("omegaconf", OmegaConf=AttrDict)
-    stub("pytorch_lightning", LightningModule=torch.nn.Module)
-    for pkg in ("enhancing", "enhancing.modules", "enhancing.modules.stage2", "enhancing.utils"):
-        stub(pkg).__path__ = []
-    stub("enhancing.utils.general", initialize_from_config=initialize_from_config)
-    stub("frozen_stub", Frozen=lambda **kw: torch.nn.Linear(2, 2))    # stands in for the cond / stage-1 models
-    s2 = os.path.join(REF, "enhancing", "modules", "stage2")
-    for name in ("layers", "transformer"):
-        spec = importlib.util.spec_from_file_location(f"enhancing.modules.stage2.{name}", os.path.join(s2, f"{name}.py"))
-        mod = importlib.util.module_from_spec(spec)
-        monkeypatch.setitem(sys.modules, spec.name, mod)
-        spec.loader.exec_module(mod)
-        if name == "layers":
-            ref_gpt = mod.GPT
-            etb.patch_stage2(mod)                               # before transformer.py does `from .layers import *`
-            assert mod.GPT is etb.GPT and mod.GPT is not ref_gpt
-    tr = sys.modules["enhancing.modules.stage2.transformer"]
-    gpt_cfg = AttrDict(target="enhancing.modules.stage2.layers.GPT",
-                       params=dict(vocab_cond_size=10, vocab_img_size=64, embed_dim=64, cond_num_tokens=1, img_num_tokens=16, n_heads=2, n_layers=2))
-    frozen = AttrDict(target="frozen_stub.Frozen", params={})
-    model = tr.CondTransformer(cond_key="class", cond=frozen, stage1=frozen, transformer=gpt_cfg)
-    assert isinstance(model.transformer, etb.GPT)
-    model.learning_rate = 1e-4
-    (optimizer,), _ = model.configure_optimizers()
-    n_opt = sum(len(g["params"]) for g in optimizer.param_groups)
-    assert n_opt == len(list(model.transformer.parameters()))
-    decay = {id(p) for p in optimizer.param_groups[0]["params"]}
-    assert id(model.transformer.head.weight) in decay and id(model.transformer.blocks[0].attn.time_mix) not in decay
+    from oracle.gen_golden_live import GPT_ABI_CFG
+    layers = types.ModuleType("stage2_layers_stand_in")
+    layers.GPT = object
+    etb.patch_stage2(layers)
+    assert layers.GPT is etb.GPT
+    gpt = getattr(layers, "GPT")(**GPT_ABI_CFG)
+    assert isinstance(gpt, etb.GPT)
+    kinds = (torch.nn.Linear, torch.nn.LayerNorm, torch.nn.Embedding)
+    owners = []
+    for mn, m in gpt.named_modules():
+        for pn, _ in m.named_parameters(recurse=False):
+            kind = next((k.__name__ for k in kinds if isinstance(m, k)), "other")
+            owners.append(f"{mn + '.' if mn else ''}{pn}:{kind}")
+    want = np.load(os.path.join(golden_dir, "ref_modules.npz"))["gptabi.owners"].tolist()
+    assert sorted(owners) == want, set(owners) ^ set(want)
 
 
 def test_c_abi_rejects_bad_arguments_before_touching_the_device():

@@ -475,82 +475,74 @@ def test_frozen_model_backward_skips_parameter_gradients():
     assert n_frozen < etb.ops.launch_count() - n0
 
 
-def test_non_square_patches_match_the_reference_modules():
-    """reference layers.py:157-166 accepts (height, width) patches; checked against the vendored reference modules
-    (oracle/_ref, built by oracle/build_ref.py) on the CPU"""
-    import importlib.util
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "enhancing_ref")
-    if not os.path.exists(os.path.join(ref_dir, "layers.py")):
-        pytest.skip("oracle/_ref not present")
-    if not hasattr(np, "float"):
-        np.float = float
-    spec = importlib.util.spec_from_file_location("enhancing_ref_ns.layers", os.path.join(ref_dir, "layers.py"))
-    RL = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(RL)
+def test_non_square_patches_match_the_reference_modules(golden_dir):
+    """reference layers.py:157-166 accepts (height, width) patches; checked against the reference's own modules
+    (tests/golden/ref_modules.npz, oracle/gen_golden_live.py: outputs as strided samples, the reference's positional tables)"""
+    from oracle.gen_golden_live import NONSQUARE_KW as kw
+    from oracle.seeded import parse_shapes, seeded_state_dict, strided_sample
+    g = np.load(os.path.join(golden_dir, "ref_modules.npz"))
     etb.set_precision("parity")
-    torch.manual_seed(0)
-    kw = dict(image_size=(32, 48), patch_size=(8, 4), dim=64, depth=1, heads=2, mlp_dim=128, dim_head=32)
-    ref_e, ref_d = RL.ViTEncoder(**kw), RL.ViTDecoder(**kw)
     enc, dec = etb.ViTEncoder(**kw), etb.ViTDecoder(**kw)
-    enc.load_state_dict(ref_e.state_dict(), strict=True); dec.load_state_dict(ref_d.state_dict(), strict=True)
+    for tag, m, pos in (("enc", enc, "en_pos_embedding"), ("dec", dec, "de_pos_embedding")):
+        sd = seeded_state_dict(parse_shapes(g[f"nonsquare.{tag}.shapes"]), seed=11)
+        sd[pos] = torch.from_numpy(g["nonsquare." + pos])
+        m.load_state_dict(sd, strict=True)
     enc.cuda(); dec.cuda()
-    img = torch.rand(2, 3, 32, 48)
-    h_ref = ref_e(img)
-    rec_ref = ref_d(h_ref)
+    img = torch.rand(2, 3, 32, 48, generator=torch.Generator().manual_seed(0))
     h = enc(img.cuda())
-    assert h.shape == h_ref.shape == (2, 48, 64)
-    assert relmax(h.cpu(), h_ref.detach()) < 5e-5
-    assert relmax(dec(h).cpu(), rec_ref.detach()) < 5e-5
+    assert h.shape == (2, 48, 64)
+
+    def rel(a, key):
+        return ((strided_sample(a.detach().cpu(), 2048).double() - torch.from_numpy(g[key]).double()).abs().max()
+                / float(g[key + "_absmax"])).item()
+    assert rel(h, "nonsquare.h") < 5e-5
+    assert rel(dec(h), "nonsquare.rec") < 5e-5
     with pytest.raises(NotImplementedError, match="multiple of 4"):
         etb.ViTEncoder(image_size=30, patch_size=6, dim=64, depth=1, heads=2, mlp_dim=64)
 
 
 @pytest.mark.parametrize("residual", [False, True])
-def test_gumbel_quantizer_matches_reference(residual):
+def test_gumbel_quantizer_matches_reference(golden_dir, residual):
     """reference quantizers.py:95-126 (SURVEY.md section 8 f-4).  The quantiser is stochastic; with the generator seeded
     identically F.gumbel_softmax draws the same noise on the same device, so the soft sample, the KL loss and the
-    gradients of the vendored reference class (oracle/_ref, moved to the GPU, TF32 matmuls off) are reproduced up to
-    the rounding of the logits; in eval mode (hard one-hot of a noisy arg-max) the indices agree except at near-ties."""
-    import importlib.util
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "enhancing_ref")
-    if not os.path.exists(os.path.join(ref_dir, "quantizers.py")):
-        pytest.skip("oracle/_ref not present")
-    spec = importlib.util.spec_from_file_location("enhancing_ref_ns.quantizers", os.path.join(ref_dir, "quantizers.py"))
-    RQ = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(RQ)
+    gradients the reference class produced on a B200 with TF32 matmuls off (tests/golden/gumbel_cuda.npz,
+    oracle/gen_golden_live.py --gumbel: strided samples) are reproduced up to the rounding of the logits; in eval mode (hard
+    one-hot of a noisy arg-max) the indices agree except at near-ties."""
+    from oracle.gen_golden_live import GUMBEL_KW
+    from oracle.seeded import seeded_state_dict, strided_sample
+    g = np.load(os.path.join(golden_dir, "gumbel_cuda.npz"))
+    tag = "res3" if residual else "plain"
     torch.backends.cuda.matmul.allow_tf32 = False
-    kw = dict(embed_dim=32, n_embed=512, temp_init=0.7, use_residual=residual, num_quantizers=3 if residual else None)
-    torch.manual_seed(0)
-    ref = RQ.GumbelQuantizer(**kw).cuda()
-    ours = etb.GumbelQuantizer(**kw).cuda()
-    ours.load_state_dict(ref.state_dict(), strict=True)
-    z0 = torch.randn(2, 96, 32, device="cuda")
+    ours = etb.GumbelQuantizer(use_residual=residual, num_quantizers=3 if residual else None, **GUMBEL_KW)
+    ours.load_state_dict(seeded_state_dict({k: tuple(p.shape) for k, p in ours.named_parameters()}, seed=5), strict=True)
+    ours.cuda()
+    z0 = torch.randn(2, 96, 32, generator=torch.Generator().manual_seed(6)).cuda()
+
+    def rel(a, key):
+        return ((strided_sample(a.detach().cpu(), 2048).double() - torch.from_numpy(g[key]).double()).abs().max()
+                / float(g[key + "_absmax"])).item()
     # training mode: soft samples, gradients through the sample
-    outs = []
-    for q in (ref, ours):
-        q.train(); q.zero_grad()
-        z = z0.clone().requires_grad_(True)
-        torch.manual_seed(123)
-        zq, loss, idx = q(z)
-        (zq.square().mean() + loss).backward()
-        outs.append((zq.detach(), loss.detach(), idx, z.grad, q.embedding.weight.grad.clone()))
-    (zq_r, l_r, i_r, gz_r, ge_r), (zq_o, l_o, i_o, gz_o, ge_o) = outs
-    assert zq_o.shape == zq_r.shape and i_o.shape == i_r.shape and i_o.dtype == torch.int64
-    assert relmax(zq_o, zq_r) < 2e-4 and abs(float(l_o - l_r)) < 1e-5 * max(1.0, abs(float(l_r)))
-    assert (i_o == i_r).float().mean() > 0.99
-    if gz_r is None:          # residual mode quantises a detached copy of z (quantizers.py:43) and has no straight-through term
-        assert gz_o is None
+    ours.train()
+    z = z0.clone().requires_grad_(True)
+    torch.manual_seed(123)
+    zq_o, l_o, i_o = ours(z)
+    (zq_o.square().mean() + l_o).backward()
+    i_r, l_r = torch.from_numpy(g[f"{tag}.train.idx"]), float(g[f"{tag}.train.loss"])
+    assert i_o.shape == i_r.shape and i_o.dtype == torch.int64
+    assert rel(zq_o, f"{tag}.train.zq") < 2e-4 and abs(l_o.item() - l_r) < 1e-5 * max(1.0, abs(l_r))
+    assert (i_o.cpu() == i_r).float().mean() > 0.99
+    if f"{tag}.train.gz" not in g.files:      # residual mode quantises a detached copy of z (quantizers.py:43) and has no straight-through term
+        assert z.grad is None
     else:
-        assert relmax(gz_o, gz_r) < 2e-3
-    assert relmax(ge_o, ge_r) < 2e-3
-    # eval mode: hard samples
+        assert rel(z.grad, f"{tag}.train.gz") < 2e-3
+    assert rel(ours.embedding.weight.grad, f"{tag}.train.ge") < 2e-3
+    # eval mode: hard samples (every third token stored)
+    ours.eval()
+    torch.manual_seed(7)
     with torch.no_grad():
-        res = []
-        for q in (ref, ours):
-            q.eval()
-            torch.manual_seed(7)
-            res.append(q(z0))
-    assert (res[0][2] == res[1][2]).float().mean() > 0.99
-    same = (res[0][2] == res[1][2])
+        zq_o, _, i_o = ours(z0)
+    i_r = torch.from_numpy(g[f"{tag}.eval.idx"])
+    assert (i_o.cpu() == i_r).float().mean() > 0.99
+    same = (i_o.cpu() == i_r)[:, ::3]
     same = same.all(-1) if residual else same
-    assert relmax(res[1][0][same], res[0][0][same]) < 1e-4
+    assert relmax(zq_o[:, ::3].cpu()[same], torch.from_numpy(g[f"{tag}.eval.zq"])[same]) < 1e-4

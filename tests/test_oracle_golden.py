@@ -125,46 +125,28 @@ def test_flops_match_baseline_md():
     assert abs(O.flops_per_image(O.CONFIGS["large"]) / 1e9 - 1410.1) < 0.2
 
 
-def test_oracle_matches_the_vendored_reference_modules():
-    """where oracle/_ref exists (oracle/build_ref.py: the reference's own layers.py / quantizers.py, byte for byte) the
-    oracle port is pinned against the live reference modules, fwd + bwd, on a config no fixture covers"""
-    import importlib.util
-    import pytest
-    import torch
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "enhancing_ref")
-    if not os.path.exists(os.path.join(ref_dir, "layers.py")):
-        pytest.skip("oracle/_ref not built (needs /root/reference: python oracle/build_ref.py)")
-    if not hasattr(np, "float"):
-        np.float = float
-    mods = {}
-    for name in ("layers", "quantizers"):
-        spec = importlib.util.spec_from_file_location(f"enhancing_ref_t.{name}", os.path.join(ref_dir, f"{name}.py"))
-        mods[name] = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mods[name])
-    cfg = dict(image_size=48, patch_size=8, encoder=dict(dim=64, depth=2, heads=2, mlp_dim=96, dim_head=32),
-               decoder=dict(dim=64, depth=1, heads=2, mlp_dim=64, dim_head=32),
-               quantizer=dict(embed_dim=32, n_embed=128, use_residual=True, num_quantizers=2))
+def test_oracle_matches_the_vendored_reference_modules(golden_dir):
+    """the oracle port against the reference's own layers.py / quantizers.py modules, fwd + bwd, on a config no other
+    fixture covers (tests/golden/ref_modules.npz, oracle/gen_golden_live.py: reconstruction and gradients as strided
+    samples, gradient norms in full)"""
+    from oracle.gen_golden_live import ORACLE_CFG as cfg
+    from oracle.seeded import strided_sample
+    g = _load(golden_dir, "ref_modules.npz")
     sd = O.init_vitvq_sd(cfg, seed=7)
-    e, d, q = cfg["encoder"], cfg["decoder"], cfg["quantizer"]
-    ref = dict(encoder=mods["layers"].ViTEncoder(48, 8, **e), decoder=mods["layers"].ViTDecoder(48, 8, **d),
-               quantizer=mods["quantizers"].VectorQuantizer(**q), pre_quant=torch.nn.Linear(64, 32), post_quant=torch.nn.Linear(32, 64))
-    for name, m in ref.items():
-        m.load_state_dict({k[len(name) + 1:]: v for k, v in sd.items() if k.startswith(name + ".")}, strict=True)
     img = torch.rand(2, 3, 48, 48, generator=torch.Generator().manual_seed(3))
-    quant, qloss, idx = ref["quantizer"](ref["pre_quant"](ref["encoder"](img)))
-    rec = ref["decoder"](ref["post_quant"](quant))
-    loss = ((rec - img) ** 2).mean() + qloss
-    loss.backward()
     sdg = {k: v.clone().requires_grad_(v.is_floating_point() and "pos_embedding" not in k) for k, v in sd.items()}
     loss_o, rec_o, idx_o = O.vitvq_loss(sdg, img, cfg)
     loss_o.backward()
-    assert torch.equal(idx, idx_o)
-    torch.testing.assert_close(rec_o, rec, rtol=1e-5, atol=1e-6)
-    torch.testing.assert_close(loss_o, loss, rtol=1e-6, atol=1e-8)
-    for name, m in ref.items():
-        for pn, p in m.named_parameters():
-            g = sdg[f"{name}.{pn}"].grad
-            if p.grad is None:
-                assert g is None or g.abs().max() == 0
-            else:
-                torch.testing.assert_close(g, p.grad, rtol=1e-4, atol=1e-8)
+    np.testing.assert_array_equal(idx_o.numpy(), g["oracle.idx"])
+    torch.testing.assert_close(strided_sample(rec_o.detach(), 2048), _t(g["oracle.rec"]), rtol=1e-5, atol=1e-6)
+    torch.testing.assert_close(loss_o.detach(), _t(g["oracle.loss"]), rtol=1e-6, atol=1e-8)
+    nograd = set(g["oracle.nograd"].tolist())
+    n = 0
+    for k, v in sdg.items():
+        if k in nograd:
+            assert v.grad is None or v.grad.abs().max() == 0
+            continue
+        torch.testing.assert_close(strided_sample(v.grad), _t(g["oracle.grad." + k]), rtol=1e-4, atol=1e-8, msg=lambda m, k=k: f"{k}: {m}")
+        assert abs(v.grad.double().norm().item() - float(g["oracle.gradnorm." + k])) <= 1e-4 * float(g["oracle.gradnorm." + k]) + 1e-8, k
+        n += 1
+    assert n == sum(1 for k in g.files if k.startswith("oracle.grad."))

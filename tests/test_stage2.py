@@ -1,10 +1,9 @@
 """Stage-2 transformer (SURVEY.md section 8f-3, BASELINE config 5; reference enhancing/modules/stage2/layers.py).
 
-CPU part: oracle/gpt_oracle.py against the reference-generated golden (tests/golden/gpt_tiny.npz, oracle/gen_golden_gpt.py)
-and the live vendored reference class; the replacement's module tree / state-dict keys against the golden's.
+CPU part: oracle/gpt_oracle.py against the reference-generated golden (tests/golden/gpt_tiny.npz, oracle/gen_golden_gpt.py;
+tests/golden/ref_modules.npz, oracle/gen_golden_live.py); the replacement's module tree / state-dict keys against the golden's.
 GPU part (-m gpu): the new kernels against torch fp64, and `etb.GPT` (forward, backward, sampling steps) against the golden
 and the fp64 oracle."""
-import importlib.util
 import math
 import os
 import sys
@@ -53,36 +52,27 @@ def test_gpt_oracle_sampling_steps_match_reference_golden(golden_dir):
     torch.testing.assert_close(sl, torch.from_numpy(g["sample_logits"]), rtol=1e-5, atol=1e-6)
 
 
-def _vendored_stage2():
-    path = os.path.join(ROOT, "oracle", "_ref", "enhancing_ref", "stage2_layers.py")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built (needs /root/reference: python oracle/build_ref.py)")
-    if "omegaconf" not in sys.modules:                      # imported by the reference file for a type annotation only
-        stub = types.ModuleType("omegaconf")
-        stub.OmegaConf = type("OmegaConf", (), {})
-        sys.modules["omegaconf"] = stub
-    spec = importlib.util.spec_from_file_location("enhancing_ref_t.stage2_layers", path)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
+def _seeded_gpt(golden_dir, prefix, cfg, seed, gain):
+    """etb.GPT carrying the weights the reference class ran with (oracle/seeded.py), after checking that both have the same
+    parameters"""
+    import enhancing_transformers_b200 as etb
+    from oracle.seeded import parse_shapes, seeded_state_dict
+    g = np.load(os.path.join(golden_dir, "ref_modules.npz"))
+    shapes = parse_shapes(g[prefix + "shapes"])
+    model = etb.GPT(**cfg)
+    assert {k: tuple(p.shape) for k, p in model.named_parameters()} == shapes
+    model.load_state_dict(seeded_state_dict(shapes, seed=seed, gain=gain), strict=True)
+    return g, model
 
 
-def test_gpt_oracle_matches_the_vendored_reference_class():
-    S = _vendored_stage2()
-    torch.manual_seed(3)
-    cfg = dict(vocab_cond_size=7, vocab_img_size=33, embed_dim=96, cond_num_tokens=3, img_num_tokens=21, n_heads=3, n_layers=2,
-               mlp_bias=False, attn_bias=False)                       # a config no fixture covers: no biases, 3-token prefix
-    ref = S.GPT(**cfg)
-    with torch.no_grad():
-        ref.pos_emb_code.normal_(0, 0.2)
-        ref.pos_emb_cond.normal_(0, 0.2)
-        for p in ref.parameters():
-            if p.dim() == 2:
-                p.mul_(6.0)
-    codes = torch.randint(0, 33, (2, 21))
-    conds = torch.randint(0, 7, (2, 3))
-    sd = {k: v.detach().clone() for k, v in ref.state_dict().items()}
-    torch.testing.assert_close(G.gpt_forward(sd, codes, conds, 3), ref(codes, conds).detach(), rtol=1e-5, atol=1e-6)
+def test_gpt_oracle_matches_the_vendored_reference_class(golden_dir):
+    """the oracle's forward against the reference's own GPT on a config no other fixture covers: no biases, 3-token prefix
+    (tests/golden/ref_modules.npz, oracle/gen_golden_live.py)"""
+    from oracle.seeded import parse_shapes, seeded_state_dict
+    g = np.load(os.path.join(golden_dir, "ref_modules.npz"))
+    sd = seeded_state_dict(parse_shapes(g["gptfwd.shapes"]), seed=3, gain=1.2)
+    codes, conds = torch.from_numpy(g["gptfwd.codes"]), torch.from_numpy(g["gptfwd.conds"])
+    torch.testing.assert_close(G.gpt_forward(sd, codes, conds, 3), torch.from_numpy(g["gptfwd.logits"]), rtol=1e-5, atol=1e-6)
 
 
 def test_gpt_module_tree_and_state_dict_match_reference(golden_dir):
@@ -169,31 +159,22 @@ def test_gpt_host_logic_with_emulated_kernels(golden_dir, monkeypatch, mode):
         etb.set_precision(prev)
 
 
-def test_gpt_sampler_filters_match_the_vendored_reference(monkeypatch):
+def test_gpt_sampler_filters_match_the_vendored_reference(golden_dir, monkeypatch):
     """top-k / nucleus filtering and the multinomial draw of GPT.sample (reference stage2/layers.py:228-254): with the kernels
-    emulated and the same torch RNG stream, the replacement draws the codes the live reference class draws"""
+    emulated and the same torch RNG stream, the replacement draws the codes the reference class drew
+    (tests/golden/ref_modules.npz, oracle/gen_golden_live.py)"""
     import enhancing_transformers_b200 as etb
-    S = _vendored_stage2()
+    from oracle.gen_golden_live import GPT_SAMPLE_CFG, SAMPLE_KW
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import emulated_ops
     emulated_ops.install(monkeypatch)
-    cfg = dict(vocab_cond_size=6, vocab_img_size=64, embed_dim=64, cond_num_tokens=2, img_num_tokens=9, n_heads=2, n_layers=1)
-    torch.manual_seed(7)
-    ref = S.GPT(**cfg).eval()
-    with torch.no_grad():
-        ref.pos_emb_code.normal_(0, 0.3)
-        for p in ref.parameters():
-            if p.dim() == 2:
-                p.mul_(10.0)
     prev = etb.set_precision("parity")
     try:
-        mine = etb.GPT(**cfg).eval()
-        mine.load_state_dict(ref.state_dict(), strict=True)
-        conds = torch.randint(0, 6, (3, 2))
-        for kw in (dict(top_k=7), dict(top_p=0.8), dict(top_k=12, top_p=0.6, softmax_temperature=0.7)):
-            torch.manual_seed(123)
-            with torch.no_grad():
-                l_ref, c_ref = ref.sample(conds, use_fp16=False, **kw)
+        g, mine = _seeded_gpt(golden_dir, "gptsample.", GPT_SAMPLE_CFG, seed=7, gain=1.6)
+        mine.eval()
+        conds = torch.from_numpy(g["gptsample.conds"])
+        for i, kw in enumerate(SAMPLE_KW):
+            l_ref, c_ref = torch.from_numpy(g[f"gptsample.{i}.logits"]), torch.from_numpy(g[f"gptsample.{i}.codes"])
             torch.manual_seed(123)
             l_mine, c_mine = mine.sample(conds, use_fp16=False, **kw)
             assert torch.equal(c_mine, c_ref), kw
